@@ -43,6 +43,28 @@ CONFIGS = {
 }
 SCORE_CFG = dict(n_items=500_000, d=128, seq_len=200, k=10, users_per_call=4096, sweep=(512, 4096, 32768),
                  users_per_gpu=1_048_576, distinct_histories=65_536)
+DUMP_PARAM_ELEMENTS = 1 << 23  # --dump-outputs: the fp32 parameters take at most 32 MB of its 64 MB
+
+
+def param_sample(flat):
+    """The flat parameter vector itself when it fits DUMP_PARAM_ELEMENTS, else that many elements at fixed seeded
+    positions (the same positions for the same configuration), fp32 on the host."""
+    flat = flat.detach().reshape(-1)
+    if flat.numel() > DUMP_PARAM_ELEMENTS:
+        idx = torch.randint(0, flat.numel(), (DUMP_PARAM_ELEMENTS,), generator=torch.Generator().manual_seed(0)).sort().values
+        flat = flat[idx.to(flat.device)]
+    return flat.float().cpu()
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, float32 (float64 for integer ids: exact below 2**53)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        t = t.double() if not t.is_floating_point() or t.dtype == torch.float64 else t.float()
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 def peaks():
@@ -182,7 +204,7 @@ def cpu_train_seq_per_s(c, steps=3, warmup=1):
         ts.append(time.perf_counter() - t0)
     ts = sorted(ts[warmup:])
     med = ts[len(ts) // 2]
-    return batch / med, med, float(loss.detach())
+    return batch / med, med, loss.detach(), torch.cat([p.detach().reshape(-1) for p in flat])
 
 
 def cpu_predict_users_per_s(users=64, reps=3):
@@ -213,8 +235,9 @@ def run_reference(args):
     if rank != 0:
         return
     c = CONFIGS[args.config]
-    n_timed = max(1, min(args.steps, 5 if args.config == 2 else 2))  # bounded sample: a CPU step of this workload takes seconds
-    v, med, _ = cpu_train_seq_per_s(c, steps=n_timed, warmup=1)
+    v, med, loss, flat = cpu_train_seq_per_s(c, steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"train_loss": loss.reshape(1), "train_params": param_sample(flat)})
     cores = torch.get_num_threads()
     metric = "bert4rec_train_seq_per_s" if c["kind"] == "bert" else "sasrec_train_seq_per_s"
     line = {
@@ -224,7 +247,7 @@ def run_reference(args):
         "config": {"workload": workload_string(c) + " - CPU oracle port of the reference algorithm",
                    **{k: c[k] for k in ("seq_len", "d", "heads", "blocks", "n_items")}, "global_batch": c["cpu_batch"]},
         "cpu_baseline": {"value": v, "unit": "seq/s", "cores": cores, "kind": "port",
-                         "sample": f"{n_timed} timed steps of batch {c['cpu_batch']} (fwd+bwd+Adam, dropout off), torch fp32, {cores} threads"},
+                         "sample": f"{args.steps} timed steps of batch {c['cpu_batch']} (fwd+bwd+Adam, dropout off), torch fp32, {cores} threads"},
         "e2e": {"value": v, "unit": "seq/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     if args.config == 2 and not args.no_scoring:
@@ -346,6 +369,9 @@ def run_ours(args):
     ms, loss = timed(step_dev, K)
     clocks = sampler.stop() if rank == 0 else None
     final_loss = float(loss[0].item())
+    # what the last timed step returned (loss buffer: mean CE, 1 / n_valid) and the parameters it left, before later legs
+    # overwrite both
+    outputs = {"train_loss": loss.cpu(), "train_params": param_sample(eng.p32)} if args.dump_outputs else None
     # ---- (N > 1) the gradient exchange alone: 20 back-to-back calls on the staged gradient, ranks in lock step
     exchange = None
     if world > 1:
@@ -453,7 +479,7 @@ def run_ours(args):
     if args.config == 2 and not args.no_scoring:
         del mod, core, eng, devb
         torch.cuda.empty_cache()
-        scoring = run_scoring(args, dev, rank, world, PK, barrier, time_kernel)
+        scoring = run_scoring(args, dev, rank, world, PK, barrier, time_kernel, outputs)
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()
@@ -463,7 +489,7 @@ def run_ours(args):
     step_tflops = seq_s / world * fl_seq / 1e12
     cpu = None
     if not args.no_cpu:
-        v, med, _ = cpu_train_seq_per_s(c, steps=3 if args.config == 2 else 1, warmup=1)
+        v, med, _, _ = cpu_train_seq_per_s(c, steps=3 if args.config == 2 else 1, warmup=1)
         cpu = {"value": v, "unit": "seq/s", "cores": torch.get_num_threads(), "kind": "port",
                "sample": f"timed steps of batch {c['cpu_batch']} (fwd+bwd+Adam, dropout off) of the oracle port, torch fp32 CPU"}
     line = {
@@ -492,16 +518,19 @@ def run_ours(args):
         "scoring": scoring,
         "final_loss": final_loss,
     }
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
 
 
-def run_scoring(args, dev, rank, world, PK, barrier, time_kernel):
+def run_scoring(args, dev, rank, world, PK, barrier, time_kernel, outputs=None):
     """BASELINE configs[3]: SASRec predict() top-K@10 over |I| = 500 000 with filter_seen_items, >= 1 M users per GPU.
     `value`: ids resident in HBM, engine calls (body, last-position shortcut, fused score + seen mask + top-K).
     `e2e`: pinned host ids -> ``LightningModule.predict_step`` + ``TorchTopItemsCallback(postprocessors=[SeenItemsFilter])`` ->
-    top-K ids / scores copied back to pinned host memory, every call, inside the timed region."""
+    top-K ids / scores copied back to pinned host memory, every call, inside the timed region.  ``outputs`` (a dict, or
+    None) receives the top-K ids and scores of the last device-resident call at the headline call size."""
     import torch.distributed as dist
 
     from replay_b200 import ops
@@ -555,10 +584,12 @@ def run_scoring(args, dev, rank, world, PK, barrier, time_kernel):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(n_calls):
-            call_dev(i)
+            top = call_dev(i)
         e1.record()
         barrier()
         ms_dev = maxr(e0.elapsed_time(e1))
+        if outputs is not None and Bu == sc["users_per_call"]:
+            outputs["score_topk_ids"], outputs["score_topk_scores"] = (t.cpu() for t in top)
         # end to end through the reference-facing callback
         cb = TorchTopItemsCallback(top_k=K, query_column="query_id", item_column="item_id",
                                    postprocessors=[SeenItemsFilter(item_count=I, seen_items_column="seen_ids")])
@@ -648,7 +679,14 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="sequences per GPU and step (SURVEY 8d sweeps {128, 256, 512} at config 2)")
     ap.add_argument("--dropout", type=float, default=None, help="diagnostic override of the workload's dropout; "
                     "a run with this flag is not the benchmark configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32 / "
+                         "float64, < 64 MB in all): train_loss, train_params (the updated fp32 parameters, a fixed seeded "
+                         "sample of 8 Mi elements when larger) and, with the scoring leg, score_topk_ids / score_topk_scores "
+                         "of its last call at the headline call size; the inputs are the same from run to run")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -4,7 +4,8 @@ GPU box).  TEST INFRASTRUCTURE.
     PYTHONPATH=oracle/shim:/root/reference python oracle/gen_golden.py
 
 Writes tests/golden/*.npz: seeded inputs, the reference modules' weights (state_dict) and the reference's outputs
-(hidden states, train loss, gradients, eval logits, SeenItemsFilter + torch.topk result, one Adam step).
+(hidden states, train loss, gradients, eval logits, SeenItemsFilter + torch.topk result, one Adam step).  The larger
+cases store int8-grid weights and a sample of each gradient to stay under 1 MB a file (format: oracle/golden.py).
 tests/test_oracle_golden.py checks oracle/ against these; tests/test_parity_gpu.py checks the CUDA path against them.
 """
 import os
@@ -18,6 +19,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "shim"))
 sys.path.insert(1, "/root/reference")
 warnings.filterwarnings("ignore")
+
+import golden  # noqa: E402  (oracle/golden.py, next to this script)
 
 from replay.data import FeatureHint, FeatureSource, FeatureType  # noqa: E402
 from replay.data.nn import TensorFeatureInfo, TensorFeatureSource, TensorSchema  # noqa: E402
@@ -69,19 +72,18 @@ def randomise_small_params(module, g):
                 p.add_(torch.randn(p.shape, generator=g) * 0.05)
 
 
-def sd_np(module):
-    return {"sd::" + k: v.detach().cpu().numpy().copy() for k, v in module.state_dict().items()}
-
-
-def gen_new_sasrec(tag, B, L, d, H, n_items, n_blocks, seed, with_adam=True):
+def gen_new_sasrec(tag, B, L, d, H, n_items, n_blocks, seed, with_adam=True, int8=False, grad_sample=None):
     g = torch.Generator().manual_seed(seed)
     torch.manual_seed(seed)
     pad = n_items
     model = SasRec.from_params(schema(n_items, d, pad), embedding_dim=d, num_heads=H, num_blocks=n_blocks,
                                max_sequence_length=L, dropout=0.0)
     randomise_small_params(model, g)
+    if int8:
+        golden.snap_to_int8_grid(model)
+    sd0 = {k: v.detach().clone() for k, v in model.state_dict().items()}
     ids, pmask, labels, tmask = make_batch(g, B, L, n_items, pad)
-    out = dict(sd_np(model))
+    out = golden.state_dict_arrays(model, int8)
     out.update(ids=ids.numpy(), pad_mask=pmask.numpy(), labels=labels.numpy(), target_mask=tmask.numpy(),
                n_items=n_items, d=d, H=H, L=L, n_blocks=n_blocks)
     # --- train mode: loss + grads (dropout 0)
@@ -93,7 +95,8 @@ def gen_new_sasrec(tag, B, L, d, H, n_items, n_blocks, seed, with_adam=True):
     out["train_hidden"] = res["hidden_states"][0].detach().numpy()
     out["train_loss"] = loss.detach().numpy()
     for k, p in model.named_parameters():
-        out["grad::" + k] = (p.grad if p.grad is not None else torch.zeros_like(p)).numpy().copy()
+        gr = (p.grad if p.grad is not None else torch.zeros_like(p)).numpy().copy()
+        out["grad::" + k] = golden.sample(gr, grad_sample) if grad_sample else gr
     # --- one Adam step with the reference's optimizer settings (optimizer_factory.py:56-63)
     opt = torch.optim.Adam(model.parameters(), lr=1e-3, betas=(0.9, 0.98))
     opt.step()
@@ -101,7 +104,7 @@ def gen_new_sasrec(tag, B, L, d, H, n_items, n_blocks, seed, with_adam=True):
         for k, p in model.named_parameters():
             out["adam1::" + k] = p.detach().numpy().copy()
     # restore weights for the eval leg
-    model.load_state_dict({k[4:]: torch.from_numpy(v) for k, v in out.items() if k.startswith("sd::")})
+    model.load_state_dict(sd0)
     model.eval()
     with torch.no_grad():
         inf = model(feature_tensors={"item_id": ids}, padding_mask=pmask)
@@ -129,7 +132,7 @@ def gen_legacy_sasrec(tag, B, L, d, H, n_items, n_blocks, seed):
     model = SasRecModel(schema(n_items, d, pad), num_blocks=n_blocks, num_heads=H, hidden_size=d, max_len=L, dropout=0.0)
     randomise_small_params(model, g)
     ids, pmask, labels, tmask = make_batch(g, B, L, n_items, pad)
-    out = dict(sd_np(model))
+    out = golden.state_dict_arrays(model)
     out.update(ids=ids.numpy(), pad_mask=pmask.numpy(), labels=labels.numpy(), target_mask=tmask.numpy(),
                n_items=n_items, d=d, H=H, L=L, n_blocks=n_blocks)
     model.train()
@@ -151,13 +154,15 @@ def gen_legacy_sasrec(tag, B, L, d, H, n_items, n_blocks, seed):
     print("wrote sasrec_legacy_" + tag, "loss", float(loss))
 
 
-def gen_bert4rec(tag, B, L, d, H, n_items, n_blocks, seed, tying):
+def gen_bert4rec(tag, B, L, d, H, n_items, n_blocks, seed, tying, int8=False):
     g = torch.Generator().manual_seed(seed)
     torch.manual_seed(seed)
     model = Bert4RecModel(schema(n_items, d, 0), max_len=L, hidden_size=d, num_blocks=n_blocks, num_heads=H,
                           num_passes_over_block=1, dropout=0.0, enable_positional_embedding=True,
                           enable_embedding_tying=tying)
     randomise_small_params(model, g)
+    if int8:
+        golden.snap_to_int8_grid(model)
     # left padded inputs, uniform token mask (bert4rec/dataset.py:71-92): tok False = <MASK>; pads are False too
     lens = torch.randint(2, L + 1, (B,), generator=g)
     lens[0] = L
@@ -170,7 +175,7 @@ def gen_bert4rec(tag, B, L, d, H, n_items, n_blocks, seed, tying):
     tok = (torch.rand(B, L, generator=g) > 0.3) & pmask
     tok[:, -1] = False  # make sure every row has a masked real position
     labels = ids.clone()
-    out = dict(sd_np(model))
+    out = golden.state_dict_arrays(model, int8)
     out.update(ids=ids.numpy(), pad_mask=pmask.numpy(), token_mask=tok.numpy(), labels=labels.numpy(),
                n_items=n_items, d=d, H=H, L=L, n_blocks=n_blocks, tying=int(tying))
     model.train()
@@ -466,7 +471,8 @@ def gen_reference_default_shapes():
     """The reference's OWN default / example shapes, which are not multiples of the kernels' 64-wide feature slots:
     SasRec.from_params defaults embedding_dim=192, num_heads=4 (head_dim 48; nn/sequential/sasrec/model.py:199-253), the legacy
     module's hidden_size=50, head_count=1 (sasrec/lightning.py:30-47) and SURVEY's config 1 (d=64, H=2: head_dim 32)."""
-    gen_new_sasrec("d192h4", B=4, L=12, d=192, H=4, n_items=200, n_blocks=2, seed=21, with_adam=False)
+    gen_new_sasrec("d192h4", B=4, L=12, d=192, H=4, n_items=200, n_blocks=2, seed=21, with_adam=False, int8=True,
+                   grad_sample=4096)
     gen_new_sasrec("d64h2", B=4, L=12, d=64, H=2, n_items=200, n_blocks=2, seed=22, with_adam=False)
     gen_legacy_sasrec("d50h1", B=4, L=12, d=50, H=1, n_items=200, n_blocks=2, seed=23)
 
@@ -485,10 +491,11 @@ if __name__ == "__main__":
         raise SystemExit(0)
     # shapes respect the CUDA path's tile constraints: hidden in {64,128,256,512}, head_dim in {64,128}
     gen_new_sasrec("tiny", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=11)
-    gen_new_sasrec("small", B=8, L=50, d=128, H=2, n_items=600, n_blocks=2, seed=12, with_adam=False)
+    gen_new_sasrec("small", B=8, L=50, d=128, H=2, n_items=600, n_blocks=2, seed=12, with_adam=False, int8=True,
+                   grad_sample=4096)
     gen_legacy_sasrec("tiny", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=13)
-    gen_bert4rec("tiny", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=14, tying=False)
-    gen_bert4rec("tiny_tied", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=15, tying=True)
+    gen_bert4rec("tiny", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=14, tying=False, int8=True)
+    gen_bert4rec("tiny_tied", B=6, L=16, d=64, H=1, n_items=300, n_blocks=2, seed=15, tying=True, int8=True)
     gen_seen_filter_known_answers()
     gen_dataset_layout()
     gen_sampled_losses()

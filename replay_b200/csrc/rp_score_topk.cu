@@ -473,6 +473,7 @@ RP_API int rp_seen_prepare(const int64_t* seen_ids, int n_users, int S, int item
                     int32_t* out_sorted, void* stream_) {
   using namespace rp;
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  if (!seen_ids || !out_sorted) return RP_EINVAL;
   if (n_users <= 0 || S <= 0) return RP_ESHAPE;
   if (S <= 64) seen_prepare_kernel<64><<<n_users, 64, 0, stream>>>(seen_ids, S, item_count, inv_map, out_sorted);
   else if (S <= 256) seen_prepare_kernel<256><<<n_users, 128, 0, stream>>>(seen_ids, S, item_count, inv_map, out_sorted);

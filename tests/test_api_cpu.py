@@ -266,8 +266,8 @@ def test_c_abi_argument_errors_without_a_gpu():
     assert L.rp_attn_bwd(None, None) == EINVAL and L.rp_attn_bwd(ctypes.byref(AttnBwdDesc()), None) == EINVAL
     assert L.rp_sampled_head_fwd(None, None) == EINVAL and L.rp_sampled_head_fwd(ctypes.byref(SampledDesc()), None) == EINVAL
     assert L.rp_sampled_head_bwd(ctypes.byref(SampledDesc()), None, None, None) == EINVAL
-    assert L.rp_seen_prepare(None, 1, 1, 1, None, None, None) != 0
-    assert L.rp_score_topk(None, None, None, None, 0, 1, 1, 128, 10, None, None, None, None, 0, None) != 0
+    assert L.rp_seen_prepare(None, 1, 1, 1, None, None, None) == EINVAL
+    assert L.rp_score_topk(None, None, None, None, 0, 1, 1, 128, 10, None, None, None, None, 0, None) == EINVAL
     assert L.rp_ce_head_fwd(None, None, None, None, None, 1, 1, 128, None, None, None, None, 0, None, 0, None) == EINVAL
     assert L.rp_ce_head_bwd(None, None, None, None, None, 1, 1, 128, None, None, None, None, None, 0, 0, None, 0, None) == EINVAL
     assert L.rp_ffn_fused(None, None, None, None, None, None, 1, 128, None, None) == EINVAL
@@ -509,3 +509,29 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert j["value"] > 0 and j["higher_is_better"] is True
     assert j["e2e"]["value"] == j["value"] and j["e2e"]["h2d_bytes_per_step"] == 0 and j["e2e"]["d2h_bytes_per_step"] == 0
     assert j["cpu_baseline"]["kind"] == "port" and j["cpu_baseline"]["cores"] >= 1
+
+
+def test_bench_dump_outputs_are_reproducible_and_follow_steps(tmp_path):
+    """`bench.py --dump-outputs DIR` writes what the last timed step computed as float32 / float64 .npy files (< 64 MB in
+    all); the same arguments give the same outputs (up to the order of multithreaded CPU sums), and one more timed step
+    moves the parameters by about Adam's learning rate."""
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(steps, name):
+        out = tmp_path / name
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--no-scoring", "--steps",
+                            str(steps), "--warmup", "0", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600,
+                           cwd=root)
+        assert r.returncode == 0, r.stderr[-2000:]
+        return {p.stem: np.load(p) for p in out.glob("*.npy")}
+
+    a, b, c = run(1, "a"), run(1, "b"), run(2, "c")
+    assert set(a) == {"train_loss", "train_params"}
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in a:
+        np.testing.assert_allclose(a[k], b[k], rtol=1e-5, atol=1e-7, err_msg=k)
+    assert np.abs(a["train_params"] - c["train_params"]).max() > 1e-4

@@ -5,6 +5,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden
+
 pytestmark = pytest.mark.gpu
 
 
@@ -16,8 +18,8 @@ def cuda():
 
 
 def _golden(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name))
-    return z, {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, name))
+    return z, {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
 
 
 def test_new_path_module_drop_in(golden_dir, cuda):
@@ -370,3 +372,28 @@ def test_length_bucketed_predict_matches_full_window_predict(cuda):
     hq_r = core.query_embeddings(ids_r, pm_r).float()
     core.predict_buckets = ()
     assert torch.equal(hq_r, core.query_embeddings(ids_r, pm_r).float())
+
+
+def test_bench_dump_outputs(cuda, tmp_path):
+    """`bench.py --dump-outputs DIR` on the CUDA path: the last timed step's loss buffer and parameters and the headline
+    scoring call's top-K, as float32 / float64 .npy files (< 64 MB in all), consistent with the JSON line."""
+    import json
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2", "--warmup", "0", "--no-cpu", "--no-sustained",
+                        "--no-device-batches", "--quick-scoring", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=1200, cwd=root)
+    assert r.returncode == 0, r.stderr[-2000:]
+    j = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    out = {p.stem: np.load(p) for p in tmp_path.glob("*.npy")}
+    assert set(out) == {"train_loss", "train_params", "score_topk_ids", "score_topk_scores"}
+    assert all(v.dtype in (np.float32, np.float64) for v in out.values())
+    assert sum(v.nbytes for v in out.values()) <= 64 << 20
+    assert j["steps"] == 2 and out["train_loss"][0] == np.float32(j["final_loss"])
+    assert np.isfinite(out["train_params"]).all()
+    ids, sc = out["score_topk_ids"], out["score_topk_scores"]
+    assert ids.shape == sc.shape == (4096, 10) and ids.dtype == np.float64
+    assert ((ids >= 0) & (ids < 500_000) & (ids == np.round(ids))).all() and np.isfinite(sc).all()
+    assert (np.diff(sc, axis=1) <= 0).all()

@@ -2,9 +2,10 @@
 the golden vectors of the real reference (tests/golden/bert4rec_*.npz).  Tolerances as in test_gpu_engine.py."""
 import os
 
-import numpy as np
 import pytest
 import torch
+
+from oracle import golden
 
 pytestmark = pytest.mark.gpu
 
@@ -36,8 +37,8 @@ def test_bert4rec_train_step_matches_reference(golden_dir, cuda, name):
     from oracle import bert4rec as ob
     from replay_b200.engine_bert import Bert4RecEngine, BertConfig
 
-    z = np.load(os.path.join(golden_dir, name))
-    sd = {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, name))
+    sd = {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
     P = ob.params_from_state_dict(sd)
     B, L = z["ids"].shape
     cfg = BertConfig(n_items=int(z["n_items"]), d=int(z["d"]), n_heads=int(z["H"]), n_blocks=int(z["n_blocks"]), max_len=L,
@@ -59,7 +60,7 @@ def test_bert4rec_train_step_matches_reference(golden_dir, cuda, name):
     eng.g32.zero_()
     eng.backward()
     torch.cuda.synchronize()
-    Gref = ob.params_from_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("grad::")})
+    Gref = ob.params_from_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("grad::")})
     G = eng.export_canonical(eng.grads)
     bad = []
     for (nm, a), (_, b) in zip(_flat(G), _flat(Gref)):
@@ -78,8 +79,8 @@ def test_bert4rec_predict_with_biased_head(golden_dir, cuda):
     from replay_b200 import ops
     from replay_b200.engine_bert import Bert4RecEngine, BertConfig
 
-    z = np.load(os.path.join(golden_dir, "bert4rec_tiny.npz"))
-    sd = {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, "bert4rec_tiny.npz"))
+    sd = {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
     P = ob.params_from_state_dict(sd)
     B, L = z["ids"].shape
     n_items = int(z["n_items"])
@@ -105,8 +106,8 @@ def test_bert4rec_lightning_mirror(golden_dir, cuda):
     from replay_b200.models.nn.sequential import Bert4Rec
     from replay_b200.schema import TensorFeatureInfo, TensorSchema
 
-    z = np.load(os.path.join(golden_dir, "bert4rec_tiny.npz"))
-    sd = {"_model." + k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, "bert4rec_tiny.npz"))
+    sd = {"_model." + k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
     n_items, d, H, L = int(z["n_items"]), int(z["d"]), int(z["H"]), int(z["L"])
     m = Bert4Rec(TensorSchema(TensorFeatureInfo("item_id", n_items, 0, d)), block_count=int(z["n_blocks"]), head_count=H,
                  hidden_size=d, max_seq_len=L, dropout_rate=0.0)

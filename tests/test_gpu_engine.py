@@ -11,6 +11,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden
+
 pytestmark = pytest.mark.gpu
 
 
@@ -22,8 +24,8 @@ def cuda():
 
 
 def _load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name))
-    sd = {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, name))
+    sd = {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
     return z, sd
 
 
@@ -70,13 +72,15 @@ def test_train_step_matches_reference(golden_dir, cuda, name, variant):
     eng.g32.zero_()
     eng.backward()
     torch.cuda.synchronize()
-    gref = {k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("grad::")}
+    gref = {k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("grad::")}
     Gref = osr.params_from_new_state_dict(gref) if variant == "new" else osr.params_from_legacy_state_dict(gref)
     G = eng.export_canonical(eng.grads)
     names = ["item_emb", "pos_emb"] + [f"b{i}.{k}" for i in range(len(P["blocks"])) for k in
                                        ("ln1_w", "ln1_b", "in_w", "in_b", "out_w", "out_b", "ln2_w", "ln2_b", "w1", "b1", "w2", "b2")] + ["lnf_w", "lnf_b"]
     bad = []
     for nm, a, b in zip(names, osr.flat_param_list(G), osr.flat_param_list(Gref)):
+        kept = ~b.isnan()  # large golden gradients hold a sample of their elements (oracle/golden.py)
+        a, b = a[kept], b[kept]
         if b.norm() < 1e-12:
             assert a.norm() < 1e-6, nm
             continue
@@ -85,10 +89,10 @@ def test_train_step_matches_reference(golden_dir, cuda, name, variant):
             bad.append((nm, round(c, 5), round(r, 4)))
     assert not bad, bad
     # one Adam step (lr 1e-3, betas (0.9, 0.98)): every element moves by at most lr, in the reference's direction
-    if any(k.startswith("adam1::") for k in z.files):
+    if any(k.startswith("adam1::") for k in z):
         eng.optimizer_step()
         torch.cuda.synchronize()
-        a1 = osr.params_from_new_state_dict({k[7:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("adam1::")})
+        a1 = osr.params_from_new_state_dict({k[7:]: torch.from_numpy(z[k]) for k in z if k.startswith("adam1::")})
         P1 = eng.export_canonical()
         for nm, p0, p1, r1, gr in zip(names, osr.flat_param_list(P), osr.flat_param_list(P1), osr.flat_param_list(a1),
                                       osr.flat_param_list(Gref)):

@@ -71,9 +71,10 @@ def test_score_topk_golden_reference(ops, golden_dir):
 
     import numpy as np
 
+    from oracle import golden
     from oracle import sasrec as osr
 
-    z = np.load(os.path.join(golden_dir, "sasrec_new_small.npz"))
+    z = golden.load(os.path.join(golden_dir, "sasrec_new_small.npz"))
     n_items, d = int(z["n_items"]), int(z["d"])
     table = torch.from_numpy(z["sd::body.embedder.feature_embedders.item_id.emb.weight"])[:n_items]
     hq = torch.from_numpy(z["eval_hidden_last"])

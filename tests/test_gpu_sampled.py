@@ -6,6 +6,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden
+
 pytestmark = pytest.mark.gpu
 
 
@@ -17,8 +19,8 @@ def cuda():
 
 
 def _load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name))
-    return z, {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, name))
+    return z, {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
 
 
 def _cos(a, b):

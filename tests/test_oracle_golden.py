@@ -7,14 +7,15 @@ import pytest
 import torch
 
 from oracle import bert4rec as ob
+from oracle import golden
 from oracle import sasrec as osr
 
 TOL = dict(rtol=2e-5, atol=2e-6)
 
 
 def load(golden_dir, name):
-    z = np.load(os.path.join(golden_dir, name))
-    sd = {k[4:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("sd::")}
+    z = golden.load(os.path.join(golden_dir, name))
+    sd = {k[4:]: torch.from_numpy(z[k]) for k in z if k.startswith("sd::")}
     return z, sd
 
 
@@ -30,10 +31,11 @@ def test_new_sasrec_matches_reference(golden_dir, name):
     loss, G = osr.loss_and_grads(P, ids, pm, labels, tm, H, "new")
     torch.testing.assert_close(loss, torch.from_numpy(z["train_loss"]), rtol=1e-5, atol=1e-6)
     # gradients of every parameter
-    gref = {k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("grad::")}
+    gref = {k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("grad::")}
     Gref = osr.params_from_new_state_dict(gref)
     for a, b in zip(osr.flat_param_list(G), osr.flat_param_list(Gref)):
-        torch.testing.assert_close(a, b, rtol=1e-4, atol=1e-6)
+        kept = ~b.isnan()  # large golden gradients hold a sample of their elements (oracle/golden.py)
+        torch.testing.assert_close(a[kept], b[kept], rtol=1e-4, atol=1e-6)
     # eval logits of the last position (real rows identical in eval)
     h_eval = osr.sasrec_body(P, ids, pm, H, "new", mode="eval")  # differs from train only on pad query rows
     real = pm[:, -1]
@@ -50,8 +52,8 @@ def test_new_sasrec_matches_reference(golden_dir, name):
     c = torch.from_numpy(z["candidates"])
     torch.testing.assert_close(h[:, -1] @ P["item_emb"][:n_items][c].T, torch.from_numpy(z["cand_logits"]), **TOL)
     # one Adam step (optimizer_factory.py:56-63)
-    if any(k.startswith("adam1::") for k in z.files):
-        a1 = osr.params_from_new_state_dict({k[7:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("adam1::")})
+    if any(k.startswith("adam1::") for k in z):
+        a1 = osr.params_from_new_state_dict({k[7:]: torch.from_numpy(z[k]) for k in z if k.startswith("adam1::")})
         for p, g, ref in zip(osr.flat_param_list(P), osr.flat_param_list(Gref), osr.flat_param_list(a1)):
             p1, _, _ = osr.adam_step(p, g, torch.zeros_like(p), torch.zeros_like(p), 1)
             torch.testing.assert_close(p1, ref, rtol=1e-5, atol=1e-6)
@@ -68,7 +70,7 @@ def test_legacy_sasrec_matches_reference(golden_dir, name):
     torch.testing.assert_close(h, torch.from_numpy(z["train_hidden"]), **TOL)
     loss, G = osr.loss_and_grads(P, ids, pm, labels, tm, H, "legacy")
     torch.testing.assert_close(loss, torch.from_numpy(z["train_loss"]), rtol=1e-5, atol=1e-6)
-    gref = osr.params_from_legacy_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z.files if k.startswith("grad::")})
+    gref = osr.params_from_legacy_state_dict({k[6:]: torch.from_numpy(z[k]) for k in z if k.startswith("grad::")})
     for a, b in zip(osr.flat_param_list(G), osr.flat_param_list(gref)):
         torch.testing.assert_close(a, b, rtol=1e-4, atol=1e-6)
     torch.testing.assert_close(h[:, -1] @ P["item_emb"][:n_items].T, torch.from_numpy(z["eval_logits"]), **TOL)
