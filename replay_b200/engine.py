@@ -86,6 +86,42 @@ def _ru(x, m):
     return (x + m - 1) // m * m
 
 
+def param_shapes(cfg: EncoderConfig) -> list:
+    """(name, padded shape) of every parameter, in the order of the flat buffers."""
+    d, I = cfg.dp, cfg.n_items
+    shapes = [("item_emb", (I + 1, d)), ("pos_emb", (cfg.max_len, d))]
+    for i in range(cfg.n_blocks):
+        shapes += [(f"b{i}.ln1_w", (d,)), (f"b{i}.ln1_b", (d,)), (f"b{i}.in_w", (3 * d, d)), (f"b{i}.in_b", (3 * d,)),
+                   (f"b{i}.out_w", (d, d)), (f"b{i}.out_b", (d,)), (f"b{i}.ln2_w", (d,)), (f"b{i}.ln2_b", (d,)),
+                   (f"b{i}.w1", (d, d)), (f"b{i}.b1", (d,)), (f"b{i}.w2", (d, d)), (f"b{i}.b2", (d,))]
+    return shapes + [("lnf_w", (d,)), ("lnf_b", (d,))]
+
+
+def pad_kind(name: str):
+    """(row kind, column kind) of a parameter in the padded layout: 'f' = feature axis (scattered into the head slots),
+    'f3' = three stacked feature axes (packed in-projection), None = not a feature axis."""
+    leaf = name.split(".")[-1]
+    if leaf in ("item_emb", "pos_emb"):
+        return (None, "f")
+    if leaf == "in_w":
+        return ("f3", "f")
+    if leaf == "in_b":
+        return ("f3", None)
+    if leaf in ("out_w", "w1", "w2"):
+        return ("f", "f")
+    return ("f", None)  # LayerNorm weights / biases, linear biases
+
+
+def true_shape(cfg: EncoderConfig, name: str, padded_shape) -> tuple:
+    """The reference's shape of parameter ``name`` stored with ``padded_shape``: only the axes ``pad_kind`` marks as
+    feature axes shrink (a row count such as max_len or n_items + 1 never does, whatever its value)."""
+    if not getattr(cfg, "hd_valid", 0):
+        return tuple(padded_shape)
+    true = {"f": cfg.d, "f3": 3 * cfg.d}
+    kinds = pad_kind(name)[:len(padded_shape)]
+    return tuple(x if k is None else true[k] for x, k in zip(padded_shape, kinds))
+
+
 class _CountingLib:
     """Proxy over the ctypes library that counts the sm_100a kernel launches issued through it (bench.py reports them)."""
 
@@ -125,18 +161,12 @@ class SasRecEngine:
         self.Lp = _ru(seq_len, 64)
         self.with_grad = with_grad
         self.lib = _CountingLib(lib())
-        d, I = cfg.dp, cfg.n_items   # padded width: what buffers and kernels use; cfg.d is the model's true hidden size
+        d = cfg.dp   # padded width: what buffers and kernels use; cfg.d is the model's true hidden size
         self._feat = cfg.feat_index(self.dev)
         # ---------------------------------------------------------------- flat parameter layout
-        shapes = [("item_emb", (I + 1, d)), ("pos_emb", (cfg.max_len, d))]
-        for i in range(cfg.n_blocks):
-            shapes += [(f"b{i}.ln1_w", (d,)), (f"b{i}.ln1_b", (d,)), (f"b{i}.in_w", (3 * d, d)), (f"b{i}.in_b", (3 * d,)),
-                       (f"b{i}.out_w", (d, d)), (f"b{i}.out_b", (d,)), (f"b{i}.ln2_w", (d,)), (f"b{i}.ln2_b", (d,)),
-                       (f"b{i}.w1", (d, d)), (f"b{i}.b1", (d,)), (f"b{i}.w2", (d, d)), (f"b{i}.b2", (d,))]
-        shapes += [("lnf_w", (d,)), ("lnf_b", (d,))]
         self.layout = {}
         off = 0
-        for name, shp in shapes:
+        for name, shp in param_shapes(cfg):
             n = math.prod(shp)
             self.layout[name] = (off, shp)
             off = _ru(off + n, 64)
@@ -220,18 +250,7 @@ class SasRecEngine:
 
     # ------------------------------------------------------------------------------------------------ parameters
     def _pad_kind(self, name: str):
-        """(row kind, column kind) of a parameter in the padded layout: 'f' = feature axis (scattered into the head slots),
-        'f3' = three stacked feature axes (packed in-projection), None = not a feature axis."""
-        leaf = name.split(".")[-1]
-        if leaf in ("item_emb", "pos_emb"):
-            return (None, "f")
-        if leaf == "in_w":
-            return ("f3", "f")
-        if leaf == "in_b":
-            return ("f3", None)
-        if leaf in ("out_w", "w1", "w2"):
-            return ("f", "f")
-        return ("f", None)  # LayerNorm weights / biases, linear biases
+        return pad_kind(name)
 
     def _axis_index(self, kind):
         if kind == "f":
@@ -268,8 +287,7 @@ class SasRecEngine:
         return t[rows[:, None], cols[None, :]].clone()
 
     def true_shape(self, name: str):
-        d, dp = self.cfg.d, self.cfg.dp
-        return tuple({dp: d, 3 * dp: 3 * d, 2 * dp: 2 * d}.get(x, x) for x in self.layout[name][1]) if self._hdv() else self.layout[name][1]
+        return true_shape(self.cfg, name, self.layout[name][1])
 
     def init_parameters(self, seed: int = 0):
         """Reference-style init: xavier_normal_ on >=2-D tensors, LN (1, 0), biases zero / U(+-1/sqrt(fan_in)) for the

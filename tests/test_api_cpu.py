@@ -535,3 +535,20 @@ def test_bench_dump_outputs_are_reproducible_and_follow_steps(tmp_path):
     for k in a:
         np.testing.assert_allclose(a[k], b[k], rtol=1e-5, atol=1e-7, err_msg=k)
     assert np.abs(a["train_params"] - c["train_params"]).max() > 1e-4
+
+
+@pytest.mark.parametrize("d,H,L,n_items", [(192, 4, 256, 1000), (192, 4, 512, 1000), (192, 4, 768, 1000), (64, 2, 128, 1000),
+                                           (50, 1, 128, 1000), (50, 1, 64, 127), (192, 4, 50, 255), (64, 2, 64, 383)])
+def test_true_shape_shrinks_feature_axes_only(d, H, L, n_items):
+    """The reference shape of every padded parameter: only feature axes shrink.  A row count equal to a padded width
+    (max_len or n_items + 1 in {dp, 2 dp, 3 dp}) stays what it is."""
+    from replay_b200.engine import EncoderConfig, param_shapes, true_shape
+
+    cfg = EncoderConfig(n_items=n_items, d=d, n_heads=H, n_blocks=2, max_len=L)
+    assert cfg.hd_valid > 0 and L in (cfg.dp, 2 * cfg.dp, 3 * cfg.dp) or n_items + 1 in (cfg.dp, 2 * cfg.dp, 3 * cfg.dp)
+    want = {"item_emb": (n_items + 1, d), "pos_emb": (L, d), "in_w": (3 * d, d), "in_b": (3 * d,), "out_w": (d, d),
+            "w1": (d, d), "w2": (d, d)}
+    shapes = param_shapes(cfg)
+    assert len(shapes) == 2 + 12 * 2 + 2
+    for name, padded in shapes:
+        assert true_shape(cfg, name, padded) == want.get(name.split(".")[-1], (d,)), name

@@ -218,25 +218,40 @@ def test_config5_shape_train_step_matches_oracle(cuda):
     """BASELINE configs[4] shape at a small catalog: L = 512, d = 512, H = 8 (head_dim 64), 2 blocks.  Exercises the
     512-key attention forward, the saved-probability attention backward and the d = 512 CE head against the oracle on the
     same seeded weights and batch (the reference's modules at this size would need 50 MB fixtures)."""
+    _oracle_train_step(cuda, 3, 512, 512, 8, "new", fused_attn_bwd=False)
+
+
+# the attention routes config 5 never reaches: head_dim 128 (forward <128,1>, un-fused backward, attn_last<128>), a padded
+# 128 slot (legacy hidden 100), and 257..511 keys at a small width (forward <64,2>)
+@pytest.mark.parametrize("d,H,L,variant,fused", [(128, 1, 200, "new", False), (256, 2, 256, "new", False),
+                                                 (100, 1, 128, "legacy", False), (64, 1, 300, "new", False)])
+def test_attention_route_shapes_train_step_match_oracle(cuda, d, H, L, variant, fused):
+    _oracle_train_step(cuda, 3, L, d, H, variant, fused_attn_bwd=fused)
+
+
+def _oracle_train_step(cuda, B, L, d, H, variant, fused_attn_bwd):
+    """Hidden states, loss, every gradient and the predict shortcut of a 2-block engine against the oracle on the same
+    seeded weights and batch; sequence 0 is a short history (left padding inside the window)."""
     from oracle import sasrec as osr
     from replay_b200.engine import EncoderConfig, SasRecEngine
     from replay_b200.synthetic import make_sequences
 
-    B, L, d, H, I = 3, 512, 512, 8, 1500
+    I = 1500
     P = osr.random_params(I, d, L, 2, seed=21)
     ids, pm, lab, tm = make_sequences(B, I, L, seed=5)
-    ids[0, :300], pm[0, :300] = I, False          # one short history: left padding inside a 512 window
-    lab[0, :299], tm[0, :299] = I, False
-    cfg = EncoderConfig(n_items=I, d=d, n_heads=H, n_blocks=2, max_len=L, dropout=0.0, variant="new")
+    n0 = L * 300 // 512
+    ids[0, :n0], pm[0, :n0] = I, False          # one short history: left padding inside the window
+    lab[0, :n0 - 1], tm[0, :n0 - 1] = I, False
+    cfg = EncoderConfig(n_items=I, d=d, n_heads=H, n_blocks=2, max_len=L, dropout=0.0, variant=variant)
     eng = SasRecEngine(cfg, B, L, cuda)
-    assert not eng.fused_attn_bwd
+    assert eng.fused_attn_bwd == fused_attn_bwd
     eng.load_canonical(P)
     eng.set_batch(ids.cuda(), pm.cuda(), lab.cuda(), tm.cuda())
-    hid = eng.forward_hidden_all().float().cpu().view(B, L, d)
-    ref_h = osr.sasrec_body(P, ids, pm, H, "new")
+    hid = eng.unpad_features(eng.forward_hidden_all()).float().cpu().view(B, L, d)
+    ref_h = osr.sasrec_body(P, ids, pm, H, variant)
     assert (hid - ref_h).abs().max() < 8e-2, (hid - ref_h).abs().max()
     loss = eng.forward_train()
-    ref_loss, Gref = osr.loss_and_grads(P, ids, pm, lab, tm, H, "new")
+    ref_loss, Gref = osr.loss_and_grads(P, ids, pm, lab, tm, H, variant)
     assert abs(loss[0].item() - float(ref_loss)) < 5e-3 * float(ref_loss), (loss[0].item(), float(ref_loss))
     eng.g32.zero_()
     eng.backward()
@@ -248,10 +263,10 @@ def test_config5_shape_train_step_matches_oracle(cuda):
         if c < 0.99 or abs(r - 1) > 0.04:
             bad.append((k, round(c, 5), round(r, 4)))
     assert not bad, bad
-    # predict: last hidden state through the last-position shortcut (attn_last over 512 keys)
+    # predict: last hidden state through the last-position shortcut (attn_last over all L keys)
     eng.set_batch(ids.cuda(), pm.cuda())
-    hq = eng.forward_last_hidden().float().cpu()
-    ref_e = osr.sasrec_body(P, ids, pm, H, "new", mode="eval")[:, -1]
+    hq = eng.unpad_features(eng.forward_last_hidden()).float().cpu()
+    ref_e = osr.sasrec_body(P, ids, pm, H, variant, mode="eval")[:, -1]
     assert (hq - ref_e).abs().max() < 8e-2
 
 
@@ -301,15 +316,21 @@ def test_fused_training_body_equals_unfused(cuda, variant, drop, monkeypatch):
     assert not bad, bad
 
 
-@pytest.mark.parametrize("d,H,variant,drop", [(192, 4, "new", 0.2), (50, 1, "legacy", 0.2), (64, 2, "new", 0.0)])
-def test_padded_shapes_fused_equals_unfused_and_padding_stays_zero(cuda, d, H, variant, drop, monkeypatch):
+# max_len = dp (64 / 2 heads at L = 128) and = dp (192 / 4 heads at L = 256, the reference's default width at its longest
+# fused-attention length): a row count equal to a padded width must not be taken for a feature axis
+@pytest.mark.parametrize("d,H,variant,drop,L", [pytest.param(192, 4, "new", 0.2, 32, id="192-4-new-0.2"),
+                                                pytest.param(50, 1, "legacy", 0.2, 32, id="50-1-legacy-0.2"),
+                                                pytest.param(64, 2, "new", 0.0, 32, id="64-2-new-0.0"),
+                                                pytest.param(64, 2, "new", 0.0, 128, id="64-2-new-0.0-L128"),
+                                                pytest.param(192, 4, "new", 0.2, 256, id="192-4-new-0.2-L256")])
+def test_padded_shapes_fused_equals_unfused_and_padding_stays_zero(cuda, d, H, variant, drop, L, monkeypatch):
     """Reference default shapes in padded feature slots: (1) the fused training body equals the launch-per-GEMM body;
     (2) the invariant the layout rests on - padded columns of every parameter, gradient and activation are EXACTLY zero - holds
     after real optimisation steps (a non-zero padded gradient would let Adam move padded weights away from zero)."""
     from replay_b200.engine import EncoderConfig, SasRecEngine
     from replay_b200.synthetic import make_sequences
 
-    B, L, I = 16, 32, 1000
+    B, I = 16, 1000
     cfg = EncoderConfig(n_items=I, d=d, n_heads=H, n_blocks=2, max_len=L, dropout=drop, variant=variant)
     assert cfg.hd_valid > 0
     ids, pm, lab, tm = [t.cuda() for t in make_sequences(B, I, L, seed=5)]
