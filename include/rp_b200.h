@@ -108,6 +108,25 @@ int rp_ce_head_bwd(const void* hc, const void* table, const float* bias, const i
                    float* d_bias, int fused, int n_valid_hint, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
+ * Training head: full-catalog pointwise BCE fused with the logits GEMM
+ *   replaces  BCE (BCEWithLogitsLoss(reduction="sum") / T_v against a one-hot row)   replay/nn/loss/bce.py:10-95
+ *             legacy SasRec(loss_type="BCE")._compute_loss_bce                       sasrec/lightning.py:278-308
+ *             legacy Bert4Rec(loss_type="BCE")._compute_loss_bce                     bert4rec/lightning.py:273-305
+ *   loss = (1/T_v) sum_t [ sum_i softplus(s_ti) - s_t,y_t ],  s = h.E_i + b_i (fp32), never materialised.
+ * Same conventions as rp_ce_head_*: hc / table / bias / labels / n_valid as there (n_valid in device memory: graph-capturable),
+ * d in {64, 128, 256} (512: RP_ESHAPE).  fwd: loss_out fp32 [2] = { mean BCE, 1 / n_valid } and d_hc bf16 [capacity, d]
+ * (required: one fused forward + dH pass) final after the call.  bwd (same workspace and loss_out): d_table fp32
+ * [n_items, d] and d_bias fp32 [n_items] (iff bias) are OVERWRITTEN.  n_valid_hint: load balance only (0 = unknown).
+ * ------------------------------------------------------------------------------------------------------------- */
+size_t rp_bce_head_workspace(int capacity_tokens, int n_items, int d);
+int rp_bce_head_fwd(const void* hc, const void* table, const float* bias, const int32_t* labels, const int32_t* n_valid,
+                    int capacity, int n_items, int d, float* loss_out, void* d_hc, int n_valid_hint, void* workspace,
+                    size_t workspace_bytes, void* stream);
+int rp_bce_head_bwd(const void* hc, const void* table, const float* bias, const int32_t* labels, const int32_t* n_valid,
+                    int capacity, int n_items, int d, const float* loss_out, float* d_table, float* d_bias, void* workspace,
+                    size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------------------------------------------------------
  * Transformer body.  All activations are token-major bf16 [T = B*L, d]; weights are the bf16 shadow of the fp32 masters.
  * ------------------------------------------------------------------------------------------------------------- */
 

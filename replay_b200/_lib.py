@@ -56,6 +56,9 @@ def lib():
     _sig(L.rp_ce_head_fwd, c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, c_int, P, c_size_t, P])
     _sig(L.rp_ce_head_fwd_w, c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, c_int, P, c_int, c_float, c_float, P, c_size_t, P])
     _sig(L.rp_ce_head_bwd, c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, P, c_int, c_int, P, c_size_t, P])
+    _sig(L.rp_bce_head_workspace, c_size_t, [c_int, c_int, c_int])
+    _sig(L.rp_bce_head_fwd, c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, c_int, P, c_size_t, P])
+    _sig(L.rp_bce_head_bwd, c_int, [P, P, P, P, P, c_int, c_int, c_int, P, P, P, P, c_size_t, P])
     U64, LL = ctypes.c_ulonglong, ctypes.c_longlong
     _sig(L.rp_gemm, c_int, [ctypes.POINTER(GemmDesc), P])
     _sig(L.rp_attn_fwd, c_int, [ctypes.POINTER(AttnDesc), P])

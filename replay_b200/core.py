@@ -195,13 +195,15 @@ class SasRecCore(torch.nn.Module):
     # ---- loss selection (full-catalog CE by default; sampled heads: SURVEY §8 a9)
     def set_loss(self, kind: str = "ce", **kw):
         """Remembered across engine re-creations; see SasRecEngine.set_loss."""
+        if kind == "bce" and self.cfg.dp not in (64, 128, 256):
+            raise NotImplementedError(f"the full-catalog BCE head supports padded hidden sizes 64, 128 and 256 (got {self.cfg.dp})")
         self._loss_spec = (kind, kw)
         if self.engine is not None:
             self.engine._loss_applied = None  # re-applied with the negatives' shape when the next batch is staged
             if kind in self._FULL_CATALOG:
                 self.engine.set_loss(kind, **kw)
 
-    _FULL_CATALOG = ("ce", "ce_weighted", "login_ce")   # heads over the whole catalog (no negatives)
+    _FULL_CATALOG = ("ce", "ce_weighted", "login_ce", "bce")   # heads over the whole catalog (no negatives)
 
     def _stage(self, eng, ids, pad_mask, labels, target_mask, negatives, row_weights=None):
         spec = getattr(self, "_loss_spec", ("ce", {}))

@@ -123,6 +123,37 @@ __device__ __forceinline__ float ce_ex2(float x, int q) {
   return ex2f(x);
 }
 
+// ---- element-wise terms of the full-catalog BCE head (BCEWithLogitsLoss against a one-hot row), s = h.E_i + b_i in fp32.
+// The gradient passes sum 1e4 - 1e6 sigmoids per row / column, so every term needs RELATIVE accuracy (tanh.approx-based
+// sigmoids have ~2^-11 absolute error near saturation and bias those sums): e = 2^(-|s| log2 e) on MUFU.EX2, 1 / (1 + e) on
+// MUFU.RCP, log1p(e) on the FMA pipe.  s = -inf (masked column / token) gives sigmoid 0 and softplus 0.
+__device__ __forceinline__ float rcp_approx(float x) {
+  float y;
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
+}
+// log1p(e) for e in [0, 1]: e * p(e), p a degree-7 least-squares fit of log1p(e) / e (max rel. error 3.5e-7 in fp32)
+__device__ __forceinline__ float log1p_unit(float e) {
+  float p = fmaf(e, -0.008574675768613815f, 0.044214192777872086f);
+  p = fmaf(p, e, -0.10785368084907532f);
+  p = fmaf(p, e, 0.17757023870944977f);
+  p = fmaf(p, e, -0.2449961155653f);
+  p = fmaf(p, e, 0.3327617645263672f);
+  p = fmaf(p, e, -0.49997448921203613f);
+  p = fmaf(p, e, 0.9999998211860657f);
+  return e * p;
+}
+__device__ __forceinline__ float bce_sigmoid(float s) {
+  const float e = ex2f(-fabsf(s) * kLog2e);
+  return (s >= 0.f ? 1.f : e) * rcp_approx(1.f + e);
+}
+// sigmoid(s) and softplus(s) = max(s, 0) + log1p(e^-|s|)
+__device__ __forceinline__ float bce_terms(float s, float& softplus) {
+  const float e = ex2f(-fabsf(s) * kLog2e);
+  softplus = fmaxf(s, 0.f) + log1p_unit(e);
+  return (s >= 0.f ? 1.f : e) * rcp_approx(1.f + e);
+}
+
 // ----------------------------------------------------------------------------------------------------------------
 // forward
 // ----------------------------------------------------------------------------------------------------------------
@@ -456,7 +487,14 @@ struct CeSeg {
 // pace followed them).  NI = 3 issuers take the tiles round-robin, so sub-partitions 1-3 lose a third of that each (sub-
 // partition 0 hosts the TMA thread); an mbarrier token passes the right to issue from tile to tile, which keeps the
 // instructions in tile order in the (in-order) tensor pipe.
-template <int KCH, int NSTAGE, int MODE, int NBUF, bool A_TMEM, bool INORDER, bool HAS_BIAS, int GROUPS, bool PERSIST, int TN, int CG, int NI>
+// BCE = true: the loss policy of the full-catalog BCE head (rp_bce_head_*) on the same pipeline, with other epilogues -
+//   MODE 2: G = sigmoid(s + b_i) instead of the exponential, row sums of softplus(s + b_i) instead of those of G; columns
+//           >= n_items are masked explicitly (a zero-filled item row is s = b_i, not -inf); the direct finish writes
+//           dH = acc / T_v - E[y] / T_v and the row loss sum_i softplus - s_y (no normaliser, no lse, no bound)
+//   MODE 1: G = sigmoid(s + b_row + cvec[col]) with cvec = 0 for the valid tokens and -inf beyond (the bias cannot be pulled
+//           out as a row factor e^{b_i} as it is for CE); dE = acc / T_v, d_bias = sum of G / T_v
+template <int KCH, int NSTAGE, int MODE, int NBUF, bool A_TMEM, bool INORDER, bool HAS_BIAS, int GROUPS, bool PERSIST, int TN, int CG, int NI,
+          bool BCE>
 __global__ void __launch_bounds__(64 + GROUPS * 4 * CG * 32 + (NI - 1) * 32, 1)
 ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
               const __nv_bfloat16* __restrict__ a_rows /* the row-side matrix (tmA) as a plain pointer, for A_TMEM */,
@@ -472,7 +510,7 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   // fused pass with the row tile in TMEM and no bias: the tile is multiplied by log2(e) on its way into TMEM, so a logit's
   // exponential is ONE instruction (ex2 of the accumulator word: live rows have offset 0) instead of FFMA + ex2 - the
   // epilogue warps next to the MMA-issuing thread are short of issue slots (profiles/r2_ce_timeline.md)
-  constexpr bool PRESCALE = FUSED && A_TMEM && !HAS_BIAS && (RP_CE_PRESCALE != 0);
+  constexpr bool PRESCALE = FUSED && A_TMEM && !HAS_BIAS && !BCE && (RP_CE_PRESCALE != 0);
   constexpr int kEW = 4 * CG * GROUPS;   // epilogue warps in total
   constexpr int kSlots = CG * GROUPS;      // column slots of the accumulator read-out / of the row-sum partials
   static_assert(GROUPS == 1 || (GROUPS == 2 && NBUF % 2 == 0), "two epilogue warp sets: even / odd S buffers");
@@ -722,8 +760,10 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
     float crow = 0.f;
     if (MODE == 0) crow = (r0 + row < n_valid) ? cvec[r0 + row] : -INFINITY;
     if (FUSED) crow = (r0 + row < n_valid) ? (direct.use_lse_off ? -direct.lse[r0 + row] * kLog2e : 0.f) : -INFINITY;
-    float zacc = 0.f;  // FUSED: sum of G~ over this thread's columns
+    float zacc = 0.f;  // FUSED: sum of G~ over this thread's columns (BCE: of softplus)
     float gsum = 0.f;  // COL mode with bias: sum over tokens of G (before the e^{b_i} row factor) -> bias gradient
+    // BCE, COL mode: the item's bias enters every logit of the row (rows beyond the catalog are never written)
+    const float brow = (BCE && COLCONST && HAS_BIAS && r0 + row < n_items) ? bias[r0 + row] : 0.f;
     if (A_TMEM) {
       // thread (row, column group) copies its slice of the row tile from global memory into TMEM: K elements
       // [cg*D/CG, (cg+1)*D/CG) of row r0+row -> packed columns [cg*D/(2CG), ...); rows beyond the matrix read as zero
@@ -796,7 +836,20 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         constexpr int EVERY = decltype(every_c)::value;
         uint32_t pk[CW / 2];
         const int col0 = (jg0 + j) * TN + cg * kW + k * CW;
-        if (COLCONST) {
+        if (COLCONST && BCE) {
+          const float4* cc = reinterpret_cast<const float4*>(&s_cc[s][cg * kW + k * CW]);
+#pragma unroll
+          for (int q = 0; q < CW; q += 4) {
+            const float4 o = cc[q >> 2];   // 0 (valid token) or -inf
+            const float g0_ = bce_sigmoid(__uint_as_float(raw[q + 0]) + brow + o.x);
+            const float g1_ = bce_sigmoid(__uint_as_float(raw[q + 1]) + brow + o.y);
+            const float g2_ = bce_sigmoid(__uint_as_float(raw[q + 2]) + brow + o.z);
+            const float g3_ = bce_sigmoid(__uint_as_float(raw[q + 3]) + brow + o.w);
+            if (HAS_BIAS) gsum += (g0_ + g1_) + (g2_ + g3_);
+            pk[(q >> 1) + 0] = pack_bf16(g0_, g1_);
+            pk[(q >> 1) + 1] = pack_bf16(g2_, g3_);
+          }
+        } else if (COLCONST) {
           const float4* cc = reinterpret_cast<const float4*>(&s_cc[s][cg * kW + k * CW]);
 #pragma unroll
           for (int q = 0; q < CW; q += 4) {
@@ -823,7 +876,24 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
               sv[q + 3] += b4.w;
             }
           }
-          if (col0 + CW <= n_items) {  // (warp-uniform) every column of this chunk exists: no per-element masking in the hot loop
+          if (BCE) {
+            if (col0 + CW > n_items) {  // (warp-uniform) ragged last tile: the missing items' zero rows would give s = b_i
+#pragma unroll
+              for (int q = 0; q < CW; ++q)
+                if (col0 + q >= n_items) sv[q] = -INFINITY;
+            }
+            float z0 = 0.f, z1 = 0.f;
+#pragma unroll
+            for (int q = 0; q < CW; q += 2) {
+              float sp0, sp1;
+              const float g0_ = bce_terms(sv[q + 0], sp0);
+              const float g1_ = bce_terms(sv[q + 1], sp1);
+              z0 += sp0;
+              z1 += sp1;
+              pk[q >> 1] = pack_bf16(g0_, g1_);
+            }
+            zacc += z0 + z1;
+          } else if (col0 + CW <= n_items) {  // (warp-uniform) every column of this chunk exists: no per-element masking in the hot loop
             float z0 = 0.f, z1 = 0.f;
 #pragma unroll
             for (int q = 0; q < CW; q += 2) {
@@ -904,7 +974,8 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
     if (COLCONST) {
       float* o = reinterpret_cast<float*>(out);
       // biased head: G carries a per-item factor e^{b_i}; it was left out of the loop and is applied to the row here
-      const float rs = (HAS_BIAS && r < n_items) ? __expf(bias[r]) : 1.f;
+      // (BCE: G carries no such factor, the 1 / T_v of the mean is applied here)
+      const float rs = BCE ? loss_inv[0] : ((HAS_BIAS && r < n_items) ? __expf(bias[r]) : 1.f);
       if (HAS_BIAS) {
         s_gsum[slot][row] = gsum;
         asm volatile("bar.sync 1, %0;" ::"r"(kEW * 32) : "memory");  // epilogue warps only
@@ -946,7 +1017,7 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       const float inv_n = n_valid > 0 ? 1.f / (float)n_valid : 0.f;
       const int y = live ? labels[r] : 0;
       float wg = (live && direct.row.w_ext) ? direct.row.w_ext[r] : 1.f;   // gradient weight of the row
-      if (direct.row.kind == 1) {
+      if (!BCE && direct.row.kind == 1) {
         // LogInCE: the weight needs the target logit before the gradient can be scaled - one extra pass over h . E[y]
         float dp = 0.f;
         if (live) {
@@ -974,8 +1045,8 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         float rl_unused;
         if (live) ce_row_terms(direct.row, r, __logf(z) - crow * kLn2, zy0, rl_unused, wg);
       }
-      const float scale = live ? wg * inv_n / z : 0.f;
-      const float lab = wg * inv_n;
+      const float scale = live ? (BCE ? inv_n : wg * inv_n / z) : 0.f;   // BCE: G is final, no normaliser
+      const float lab = BCE ? inv_n : wg * inv_n;
       float dot = 0.f;
 #pragma unroll 1
       for (int c = 0; c < DW; c += 16) {
@@ -1012,6 +1083,9 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
           for (int k = 0; k < kSlots; ++k) zy += s_dot[k][row];
           if (HAS_BIAS) zy += bias[y];
+          if (BCE) {   // row loss: sum_i softplus(s_i) - s_y (the dE pass's token mask is written by the loss reduction)
+            direct.row_loss[r] = z - zy;
+          } else {
           const float lse2 = log2f(z) - crow;   // (crow = 0 unless the pass runs behind the two-pass forward)
           float rl, wg2;
           ce_row_terms(direct.row, r, lse2 * kLn2, zy, rl, wg2);
@@ -1019,7 +1093,8 @@ ce_bwd_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           direct.cvec[r] = -lse2 + log2f(wg2 * inv_n);
           direct.row_loss[r] = rl;
           if (direct.row.roww) direct.row.roww[r] = wg2;
-        } else {
+          }
+        } else if (!BCE) {
           direct.cvec[r] = -INFINITY;  // rows beyond T_v contribute nothing to the dE pass
         }
       }
@@ -1291,6 +1366,105 @@ static int wide_chunk_rows(int cap, int n_items) {
   return (int)rows;
 }
 
+// ---- full-catalog BCE head: completion of the fused pass
+// n_splits == 1 (the fused kernel wrote dH and the row losses): mean loss over the valid targets in a fixed order, 1 / T_v,
+// and the dE pass's token mask (0 for t < T_v, -inf up to the padded capacity)
+__global__ void __launch_bounds__(1024) bce_loss_reduce_kernel(const float* __restrict__ row_loss,
+                                                               const int32_t* __restrict__ n_valid_ptr, int cap128,
+                                                               float* __restrict__ mask, float* __restrict__ loss_out) {
+  __shared__ float red[1024];
+  const int n_valid = *n_valid_ptr;
+  float a = 0.f;
+  for (int i = threadIdx.x; i < n_valid; i += 1024) a += row_loss[i];
+  for (int i = threadIdx.x; i < cap128; i += 1024) mask[i] = i < n_valid ? 0.f : -INFINITY;
+  red[threadIdx.x] = a;
+  __syncthreads();
+  for (int o = 512; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const float inv_n = n_valid > 0 ? 1.f / (float)n_valid : 0.f;
+    loss_out[0] = red[0] * inv_n;
+    loss_out[1] = inv_n;
+  }
+}
+
+// n_splits > 1: reduce the column splits.  One warp per token:  dHc[t] = (sum_p dH~_p[t] - E[y_t]) / T_v,
+// row loss = sum of the softplus partials - s_y (fp32 gather-dot, + b_y); the token mask as above; deterministic loss sum
+// (per-block partials, the last block adds them in index order)
+__global__ void bce_finalize_kernel(const float* __restrict__ part_dh, const float* __restrict__ zpart,
+                                    const __nv_bfloat16* __restrict__ hc, const __nv_bfloat16* __restrict__ table,
+                                    const int32_t* __restrict__ labels, const float* __restrict__ bias,
+                                    const int32_t* __restrict__ n_valid_ptr, int n_splits, int z_slots, int capacity, int cap128,
+                                    int d, __nv_bfloat16* __restrict__ d_hc, float* __restrict__ mask,
+                                    float* __restrict__ block_sums, unsigned int* __restrict__ ticket,
+                                    float* __restrict__ loss_out) {
+  const int n_valid = *n_valid_ptr;
+  const float inv_n = n_valid > 0 ? 1.f / (float)n_valid : 0.f;
+  const int lane = threadIdx.x & 31, wpb = blockDim.x >> 5;
+  float local = 0.f;
+  for (int t = blockIdx.x * wpb + (threadIdx.x >> 5); t < cap128; t += gridDim.x * wpb) {
+    if (t >= n_valid || t >= capacity) {
+      if (lane == 0) mask[t] = -INFINITY;
+      continue;
+    }
+    float z = 0.f;
+    for (int i = lane; i < n_splits * z_slots; i += 32) z += zpart[(size_t)i * capacity + t];
+    const int y = labels[t];
+    const __nv_bfloat16* hr = hc + (size_t)t * d;
+    const __nv_bfloat16* er = table + (size_t)y * d;
+    float dot = 0.f;
+    for (int c = lane * 4; c < d; c += 128) {
+      const uint2 hraw = *reinterpret_cast<const uint2*>(hr + c), eraw = *reinterpret_cast<const uint2*>(er + c);
+      const float2 h0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hraw.x));
+      const float2 h1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hraw.y));
+      const float2 e0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&eraw.x));
+      const float2 e1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&eraw.y));
+      dot = fmaf(h0.x, e0.x, fmaf(h0.y, e0.y, fmaf(h1.x, e1.x, fmaf(h1.y, e1.y, dot))));
+      float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll 8
+      for (int p = 0; p < n_splits; ++p) {
+        const float4 v = __ldg(reinterpret_cast<const float4*>(part_dh + ((size_t)p * capacity + t) * d + c));
+        a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
+      }
+      uint2 o;
+      o.x = pack_bf16((a.x - e0.x) * inv_n, (a.y - e0.y) * inv_n);
+      o.y = pack_bf16((a.z - e1.x) * inv_n, (a.w - e1.y) * inv_n);
+      *reinterpret_cast<uint2*>(d_hc + (size_t)t * d + c) = o;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      z += __shfl_xor_sync(0xffffffffu, z, o);
+      dot += __shfl_xor_sync(0xffffffffu, dot, o);
+    }
+    if (bias) dot += bias[y];
+    if (lane == 0) {
+      mask[t] = 0.f;
+      local += z - dot;
+    }
+  }
+  __shared__ float red[32];
+  __shared__ bool last;
+  if (lane == 0) red[threadIdx.x >> 5] = local;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float sum = 0.f;
+    for (int i = 0; i < wpb; ++i) sum += red[i];
+    block_sums[blockIdx.x] = sum;
+    __threadfence();
+    last = (atomicAdd(ticket, 1u) == gridDim.x - 1);
+  }
+  __syncthreads();
+  if (last && threadIdx.x == 0) {
+    __threadfence();
+    float sum = 0.f;
+    for (int i = 0; i < (int)gridDim.x; ++i) sum += reinterpret_cast<volatile float*>(block_sums)[i];
+    loss_out[0] = sum * inv_n;
+    loss_out[1] = inv_n;
+  }
+}
+
 static int pick_splits(int n_row_tiles, int n_col_tiles, int max_splits = 8) {
   const int sms = sm_count();
   int best = 1;
@@ -1386,7 +1560,7 @@ static int ce_z_slots(int d) {
   return kBwdCG * ce_groups_of(d / 64, nbuf);
 }
 
-template <int KCH, int NSTAGE, int MODE>
+template <int KCH, int NSTAGE, int MODE, bool BCE = false>
 static int launch_ce_bwd(const CUtensorMap& tmA, const void* b_mat, int b_rows, const void* a_rows, const float* cvec,
                          const int32_t* labels,
                          const void* table, const float* loss_inv, const int32_t* n_valid, int n_items, const float* bias,
@@ -1416,8 +1590,8 @@ static int launch_ce_bwd(const CUtensorMap& tmA, const void* b_mat, int b_rows, 
   // output is zeroed first because slices that end inside a row tile add their part with reductions
   constexpr bool PERSIST = (MODE == 1) && A_TMEM && (RP_CE_PERSIST != 0);
   constexpr int NI = (INORDER && RP_CE_ISSUERS > 1) ? RP_CE_ISSUERS : 1;
-  auto kern = bias ? ce_bwd_kernel<KCH, NST, MODE, NBUF, A_TMEM, INORDER, true, GROUPS, PERSIST, TN, CG, NI>
-                   : ce_bwd_kernel<KCH, NST, MODE, NBUF, A_TMEM, INORDER, false, GROUPS, PERSIST, TN, CG, NI>;
+  auto kern = bias ? ce_bwd_kernel<KCH, NST, MODE, NBUF, A_TMEM, INORDER, true, GROUPS, PERSIST, TN, CG, NI, BCE>
+                   : ce_bwd_kernel<KCH, NST, MODE, NBUF, A_TMEM, INORDER, false, GROUPS, PERSIST, TN, CG, NI, BCE>;
   RP_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   if (PERSIST) {
     RP_CUDA_CHECK(cudaMemsetAsync(out, 0, (size_t)n_items * KCH * 64 * sizeof(float), stream));
@@ -1431,7 +1605,7 @@ static int launch_ce_bwd(const CUtensorMap& tmA, const void* b_mat, int b_rows, 
   return RP_OK;
 }
 
-template <int MODE>
+template <int MODE, bool BCE = false>
 static int dispatch_ce_bwd(int d, const CUtensorMap& tmA, const void* b_mat, int b_rows, const void* a_rows, const float* cvec,
                            const int32_t* labels,
                            const void* table, const float* loss_inv, const int32_t* n_valid, int n_items, const float* bias,
@@ -1439,13 +1613,13 @@ static int dispatch_ce_bwd(int d, const CUtensorMap& tmA, const void* b_mat, int
                            int capacity, float* zpart, cudaStream_t stream, const CeDirect& direct = CeDirect{nullptr, nullptr, nullptr, nullptr, CeRowOpts{nullptr, nullptr, 0, 0.f, 0.f}, 0}) {
   switch (d) {
     case 64:
-      return launch_ce_bwd<1, 6, MODE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
+      return launch_ce_bwd<1, 6, MODE, BCE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
                                        safe_flag, run_if_safe, n_splits, capacity, zpart, stream, direct);
     case 128:
-      return launch_ce_bwd<2, RP_CE_NSTAGE_D128, MODE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
+      return launch_ce_bwd<2, RP_CE_NSTAGE_D128, MODE, BCE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
                                        safe_flag, run_if_safe, n_splits, capacity, zpart, stream, direct);
     case 256:
-      return launch_ce_bwd<4, 2, MODE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
+      return launch_ce_bwd<4, 2, MODE, BCE>(tmA, b_mat, b_rows, a_rows, cvec, labels, table, loss_inv, n_valid, n_items, bias, d_bias, out, grid,
                                        safe_flag, run_if_safe, n_splits, capacity, zpart, stream, direct);
     default:
       return RP_ESHAPE;
@@ -1666,6 +1840,109 @@ RP_API int rp_ce_head_bwd(const void* hc, const void* table, const float* bias, 
   if (rc != RP_OK) return rc;
   ce_label_scatter_kernel<<<sm_count() * 4, 256, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(hc), labels, loss_inv,
                                                                n_valid, d, d_table, d_bias, roww);
+  RP_LAUNCH_CHECK();
+  return RP_OK;
+}
+
+// ---------------------------------------------------------------------------------------------------------------------
+// Full-catalog BCE head (BCEWithLogitsLoss(reduction="sum") / T_v against a one-hot target row): the fused forward + dH pass
+// and the persistent dE pass of the CE head with the BCE epilogues (ce_bwd_kernel<..., BCE = true>).  No normaliser, so no
+// lse, no bound on |s| and no two-pass fallback.
+// workspace: [block_sums 1024 f][ticket, pad -> 64 B][zpart 16*cap f (also the row losses)][mask round_up(cap,128) f]
+//            [part_dh 8*cap*d f]
+// ---------------------------------------------------------------------------------------------------------------------
+struct BceWs {
+  float* block_sums; unsigned int* ticket; float* zpart; float* mask; float* part_dh;
+};
+static size_t bce_zpart_bytes(int cap) { return ((size_t)kMaxSplits * kBwdCG * kCeMaxGroups * cap * 4 + 255) / 256 * 256; }
+static size_t bce_mask_bytes(int cap) { return ((size_t)(cap + 127) / 128 * 128 * 4 + 255) / 256 * 256; }
+static size_t bce_ws_bytes(int cap, int d) {
+  return 4096 + 256 + bce_zpart_bytes(cap) + bce_mask_bytes(cap) + (size_t)kMaxSplits * cap * d * 4;
+}
+static BceWs bce_ws(void* workspace, int cap) {
+  uint8_t* w = reinterpret_cast<uint8_t*>(workspace);
+  BceWs r;
+  r.block_sums = reinterpret_cast<float*>(w);
+  w += 4096;
+  r.ticket = reinterpret_cast<unsigned int*>(w);
+  w += 256;
+  r.zpart = reinterpret_cast<float*>(w);
+  w += bce_zpart_bytes(cap);
+  r.mask = reinterpret_cast<float*>(w);
+  w += bce_mask_bytes(cap);
+  r.part_dh = reinterpret_cast<float*>(w);
+  return r;
+}
+
+RP_API size_t rp_bce_head_workspace(int capacity_tokens, int n_items, int d) {
+  if (capacity_tokens <= 0 || n_items <= 0 || (d != 64 && d != 128 && d != 256)) return 0;
+  return bce_ws_bytes(capacity_tokens, d);
+}
+
+// Forward + dH.  loss_out fp32 [2] = {mean BCE over the valid targets, 1 / T_v}; d_hc bf16 [capacity, d] (rows < *n_valid)
+// is final after this call.  n_valid_hint: host estimate of *n_valid (0 = unknown), load balance only.
+RP_API int rp_bce_head_fwd(const void* hc, const void* table, const float* bias, const int32_t* labels, const int32_t* n_valid,
+                           int capacity, int n_items, int d, float* loss_out, void* d_hc, int n_valid_hint, void* workspace,
+                           size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  if (!hc || !table || !labels || !n_valid || !loss_out || !d_hc || !workspace) return RP_EINVAL;
+  if (capacity <= 0 || n_items <= 0) return RP_ESHAPE;
+  if (d != 64 && d != 128 && d != 256) return RP_ESHAPE;
+  if (workspace_bytes < bce_ws_bytes(capacity, d)) return RP_EWORKSPACE;
+  const int n_tok_tiles = (capacity + kT - 1) / kT, n_item_tiles = (n_items + kT - 1) / kT;
+  const int hint_tiles = (n_valid_hint > 0 && n_valid_hint <= capacity) ? (n_valid_hint + kT - 1) / kT : n_tok_tiles;
+  BceWs ws = bce_ws(workspace, capacity);
+  CUtensorMap tmA;
+  int rc;
+  if ((rc = make_tmap_bf16(&tmA, hc, capacity, d, d, 128)) != RP_OK) return rc;
+  const int P = pick_splits(hint_tiles, n_item_tiles);
+  CeDirect direct{nullptr, nullptr, nullptr, nullptr, CeRowOpts{nullptr, nullptr, 0, 0.f, 0.f}, 0};
+  if (P == 1) {  // every CTA sees the whole catalog: dH and the row losses come straight out of the fused kernel
+    direct.d_hc = reinterpret_cast<__nv_bfloat16*>(d_hc);
+    direct.row_loss = ws.zpart;
+  }
+  rc = dispatch_ce_bwd<2, true>(d, tmA, table, n_items, hc, nullptr, labels, table, nullptr, n_valid, n_items, bias, nullptr,
+                                ws.part_dh, n_tok_tiles * P, nullptr, 1, P, capacity, ws.zpart, stream, direct);
+  if (rc != RP_OK) return rc;
+  const int cap128 = n_tok_tiles * kT;
+  if (P == 1) {
+    bce_loss_reduce_kernel<<<1, 1024, 0, stream>>>(ws.zpart, n_valid, cap128, ws.mask, loss_out);
+  } else {
+    RP_CUDA_CHECK(cudaMemsetAsync(ws.ticket, 0, 4, stream));
+    int blocks = (cap128 + 7) / 8;
+    if (blocks > 1024) blocks = 1024;
+    bce_finalize_kernel<<<blocks, 256, 0, stream>>>(ws.part_dh, ws.zpart, reinterpret_cast<const __nv_bfloat16*>(hc),
+                                                    reinterpret_cast<const __nv_bfloat16*>(table), labels, bias, n_valid, P,
+                                                    ce_z_slots(d), capacity, cap128, d, reinterpret_cast<__nv_bfloat16*>(d_hc),
+                                                    ws.mask, ws.block_sums, ws.ticket, loss_out);
+  }
+  RP_LAUNCH_CHECK();
+  return RP_OK;
+}
+
+// dE (and d_bias) of rp_bce_head_fwd for d(loss) = 1, with the SAME workspace and loss_out:
+//   d_table fp32 [n_items, d]  OVERWRITTEN with sigmoid^T . hc / T_v, then the one-hot part is atomically subtracted
+//   d_bias  fp32 [n_items] (iff bias)  OVERWRITTEN likewise
+RP_API int rp_bce_head_bwd(const void* hc, const void* table, const float* bias, const int32_t* labels, const int32_t* n_valid,
+                           int capacity, int n_items, int d, const float* loss_out, float* d_table, float* d_bias, void* workspace,
+                           size_t workspace_bytes, void* stream_) {
+  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
+  if (!hc || !table || !labels || !n_valid || !loss_out || !d_table || !workspace) return RP_EINVAL;
+  if ((bias == nullptr) != (d_bias == nullptr)) return RP_EINVAL;
+  if (capacity <= 0 || n_items <= 0) return RP_ESHAPE;
+  if (d != 64 && d != 128 && d != 256) return RP_ESHAPE;
+  if (workspace_bytes < bce_ws_bytes(capacity, d)) return RP_EWORKSPACE;
+  BceWs ws = bce_ws(workspace, capacity);
+  CUtensorMap tmE;
+  int rc;
+  if ((rc = make_tmap_bf16(&tmE, table, n_items, d, d, 128)) != RP_OK) return rc;
+  const int n_item_tiles = (n_items + kT - 1) / kT;
+  const float* loss_inv = loss_out + 1;
+  rc = dispatch_ce_bwd<1, true>(d, tmE, hc, capacity, table, ws.mask, labels, table, loss_inv, n_valid, n_items, bias, d_bias,
+                                d_table, n_item_tiles, nullptr, 0, 1, capacity, nullptr, stream);
+  if (rc != RP_OK) return rc;
+  ce_label_scatter_kernel<<<sm_count() * 4, 256, 0, stream>>>(reinterpret_cast<const __nv_bfloat16*>(hc), labels, loss_inv,
+                                                               n_valid, d, d_table, d_bias, nullptr);
   RP_LAUNCH_CHECK();
   return RP_OK;
 }

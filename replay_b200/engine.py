@@ -127,7 +127,7 @@ class _CountingLib:
 
     KERNELS = {"rp_gemm": 1, "rp_attn_fwd": 1, "rp_attn_bwd": 1, "rp_attn_last": 1, "rp_attn_softmax_bwd": 1, "rp_prepare_batch": 2, "rp_embed_fwd": 1,
                "rp_embed_bwd": 2, "rp_layernorm_fwd": 1, "rp_layernorm_bwd": 1, "rp_dropout_bwd": 1, "rp_colsum": 1, "rp_colsum_multi": 1,
-               "rp_adam_step": 2, "rp_cast_bf16": 1, "rp_counter_add": 1, "rp_reduce_splits": 1, "rp_ce_head_fwd": 2, "rp_ce_head_bwd": 3,
+               "rp_adam_step": 2, "rp_cast_bf16": 1, "rp_counter_add": 1, "rp_reduce_splits": 1, "rp_ce_head_fwd": 2, "rp_ce_head_bwd": 3, "rp_bce_head_fwd": 2, "rp_bce_head_bwd": 2,
                "rp_score_topk": 2, "rp_seen_prepare": 1, "rp_sampled_head_fwd": 4, "rp_sampled_head_bwd": 4, "rp_ffn_fused": 1, "rp_post_attn_fused": 1,
                "rp_post_attn_train": 1, "rp_wgrad_group": 2, "rp_ln_qkv_fused": 1, "rp_pre_attn_bwd": 1,
                "rp_post_attn_bwd": 1}
@@ -184,6 +184,7 @@ class SasRecEngine:
         # fused tcgen05 attention backward: head_dim 64, L <= 256; otherwise saved probabilities + batched GEMMs
         self.fused_attn_bwd = cfg.head_slot == 64 and seq_len <= 256
         self.sampled = None       # full-catalog CE unless set_loss() selects a sampled head
+        self.bce = None           # ... or the full-catalog BCE head
         self._loss_args = None
         self.fused_ffn_eval = True  # eval / predict: one-pass FFN kernel for d <= 128
         self.fused_post_attn_eval = True  # eval / predict: out-projection + LayerNorm + FFN in one kernel for d <= 128
@@ -551,6 +552,17 @@ class SasRecEngine:
         # per-row variants of the full-catalog head (rp_ce_head_fwd_w): "ce_weighted" (LogOutCEWeighted / CEWeighted: sample
         # weights staged with set_row_weights) and "login_ce" (LogInCE); "ce" is the plain head
         self.ce_row = None
+        self.bce = None
+        if kind == "bce":
+            # full-catalog BCE (replay/nn/loss/bce.py:10-95, legacy loss_type="BCE" without negatives): rp_bce_head_*
+            if self._dp() not in (64, 128, 256):
+                raise NotImplementedError(f"the full-catalog BCE head supports padded hidden sizes 64, 128 and 256 (got {self._dp()})")
+            self.sampled = None
+            if self.with_grad:
+                from .ops import BCEHeadState
+
+                self.bce = BCEHeadState(self.T, self.cfg.n_items, self._dp(), self.dev, loss=self.ce.loss)
+            return
         if kind in ("ce", "ce_weighted", "login_ce"):
             self.sampled = None
             if kind != "ce":
@@ -720,6 +732,12 @@ class SasRecEngine:
         if self.sampled is not None:
             check(self.lib.rp_sampled_head_fwd(ctypes.byref(self._sampled_desc()), self._stream()), "rp_sampled_head_fwd")
             return self.ce.loss
+        if self.bce is not None:
+            from .ops import bce_head_fwd
+
+            self.lib.count += 2
+            return bce_head_fwd(self.bce, self.hc, self.params16["item_emb"][: cfg.n_items], self.labels_c, self.n_valid,
+                                self.s["dhc"], n_valid_hint=self.n_valid_hint)
         from .ops import ce_head_fwd
 
         self.lib.count += 2
@@ -750,6 +768,11 @@ class SasRecEngine:
             G["item_emb"].zero_()  # the sampled head accumulates sparse rows (the full-CE head overwrites the dense table)
             check(self.lib.rp_sampled_head_bwd(ctypes.byref(self._sampled_desc()), s["dhc"].data_ptr(), G["item_emb"].data_ptr(),
                                                st()), "rp_sampled_head_bwd")
+        elif self.bce is not None:
+            from .ops import bce_head_bwd
+
+            bce_head_bwd(self.bce, self.hc, p16["item_emb"][: cfg.n_items], self.labels_c, self.n_valid, G["item_emb"])
+            self.lib.count += 2
         else:
             ce_head_bwd(self.ce, self.hc, p16["item_emb"][: cfg.n_items], self.labels_c, self.n_valid, s["dhc"], G["item_emb"],
                         n_valid_hint=self.n_valid_hint)

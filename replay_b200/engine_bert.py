@@ -92,7 +92,7 @@ class Bert4RecEngine(SasRecEngine):
         self.params16 = {k: self.p16[o:o + math.prod(s)].view(s) for k, (o, s) in self.layout.items()}
         if with_grad:
             self._alloc_grad_state()
-        self.sampled, self._loss_args = None, None
+        self.sampled, self._loss_args, self.bce = None, None, None
         self.rng_counter = torch.zeros(1, device=self.dev, dtype=torch.int64)
         self.seed = seed & 0xFFFFFFFFFFFF
         self.fused_attn_bwd = (cfg.d // cfg.n_heads) == 64 and seq_len <= 256
@@ -277,8 +277,23 @@ class Bert4RecEngine(SasRecEngine):
         W16 = self.params16["item_emb"] if cfg.tying else self.params16["head_w"]
         return W16, self.params["head_b"]
 
+    def set_loss(self, kind: str = "ce", **kw):
+        """``"ce"`` (default) or ``"bce"``: full-catalog CE / pointwise BCE (bert4rec/lightning.py:273-305) over the biased
+        (or tied + out_bias) head.  The sampled losses of the reference's BERT4Rec are not built."""
+        if kind not in ("ce", "bce"):
+            raise NotImplementedError(f"Not supported loss_type {kind!r}")
+        self._loss_args = (kind, kw)
+        self.bce = None
+        if kind == "bce":
+            if self.cfg.d not in (64, 128, 256):
+                raise NotImplementedError(f"the full-catalog BCE head supports hidden sizes 64, 128 and 256 (got {self.cfg.d})")
+            if self.with_grad:
+                from .ops import BCEHeadState
+
+                self.bce = BCEHeadState(self.T, self.cfg.n_items, self.cfg.d, self.dev, loss=self.ce.loss)
+
     def forward_train(self):
-        from .ops import ce_head_fwd
+        from .ops import bce_head_fwd, ce_head_fwd
 
         self._prepare(True)
         self._body_forward(True)
@@ -286,12 +301,15 @@ class Bert4RecEngine(SasRecEngine):
                                       self.cfg.d, self.hc.data_ptr(), 0, self._stream()), "rp_gather_rows")
         W16, bias = self._head()
         self.lib.count += 2
+        if self.bce is not None:
+            return bce_head_fwd(self.bce, self.hc, W16, self.labels_c, self.n_valid, self.s["dhc"], bias=bias,
+                                n_valid_hint=self.n_valid_hint)
         return ce_head_fwd(self.ce, self.hc, W16, self.labels_c, self.n_valid, bias=bias,
                            d_hc=self.s["dhc"] if self.fused_ce else None, n_valid_hint=self.n_valid_hint)
 
     # ------------------------------------------------------------------------------------------------ backward
     def backward(self):
-        from .ops import ce_head_bwd
+        from .ops import bce_head_bwd, ce_head_bwd
 
         cfg, T, d, L = self.cfg, self.T, self.cfg.d, self.L
         p16, prm, G, s = self.params16, self.params, self.grads, self.s
@@ -302,8 +320,12 @@ class Bert4RecEngine(SasRecEngine):
         st, rng = self._stream, self.rng_counter.data_ptr()
         W16, bias = self._head()
         dW = G["item_emb"] if cfg.tying else G["head_w"]
-        ce_head_bwd(self.ce, self.hc, W16, self.labels_c, self.n_valid, s["dhc"], dW, bias=bias, d_bias=G["head_b"])
-        self.lib.count += 3
+        if self.bce is not None:
+            bce_head_bwd(self.bce, self.hc, W16, self.labels_c, self.n_valid, dW, bias=bias, d_bias=G["head_b"])
+            self.lib.count += 2
+        else:
+            ce_head_bwd(self.ce, self.hc, W16, self.labels_c, self.n_valid, s["dhc"], dW, bias=bias, d_bias=G["head_b"])
+            self.lib.count += 3
         dx = s["dxa"]
         dx.zero_()
         check(self.lib.rp_gather_rows(s["dhc"].data_ptr(), self.valid_idx.data_ptr(), T, self.n_valid.data_ptr(), d,

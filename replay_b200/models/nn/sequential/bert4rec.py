@@ -97,8 +97,19 @@ class _BertCore(SasRecCore):
                     out[prefix + "_head._item_embedder." + k[len("item_embedder."):]] = v
         return out
 
+    def _apply_loss(self, eng) -> bool:
+        """Select the engine's head for the remembered loss ("ce" | "bce"); True when it changed (captured graphs are stale)."""
+        spec = getattr(self, "_loss_spec", ("ce", {}))
+        key = (spec[0], tuple(sorted(spec[1].items())))
+        if getattr(eng, "_loss_applied", None) == key:
+            return False
+        eng.set_loss(spec[0], **spec[1])
+        eng._loss_applied = key
+        return True
+
     def loss(self, ids, pad_mask, token_mask, labels):
         eng = self.ensure_engine(*ids.shape, with_grad=True)
+        self._apply_loss(eng)
         eng.set_batch(ids, pad_mask, token_mask, labels)
         return _EngineLoss.apply(self.flat, self)
 
@@ -107,6 +118,8 @@ class _BertCore(SasRecCore):
         if self._shadow_dirty:
             eng.refresh_shadow(); self._shadow_dirty = False
         self._set_lr(eng, lr)
+        if self._apply_loss(eng):
+            self._drop_graphs()   # another loss head: different kernels / buffers
         eng.set_batch(ids, pad_mask, token_mask, labels)
         if isinstance(all_reduce, str):
             return self._graph_trainer(eng).run()[0]
@@ -183,13 +196,16 @@ class Bert4Rec(LightningModuleBase):
                  lr_scheduler_factory=None, fused_optimizer: bool = True, device=None):
         super().__init__()
         self.save_hyperparameters()
-        if loss_type != "CE" or loss_sample_count is not None:
-            raise NotImplementedError("Not supported loss_type")
+        if loss_type not in ("CE", "BCE") or loss_sample_count is not None:
+            raise NotImplementedError("Not supported loss_type")   # sampled losses / CE_restricted: no fused head
         self._model = Bert4RecModel(tensor_schema, max_len=max_seq_len, hidden_size=hidden_size, num_blocks=block_count,
                                     num_heads=head_count, num_passes_over_block=pass_per_transformer_block_count,
                                     dropout=dropout_rate, enable_positional_embedding=enable_positional_embedding,
                                     enable_embedding_tying=enable_embedding_tying, device=device)
         self._schema = tensor_schema
+        self._loss_type = loss_type
+        if loss_type == "BCE":   # full-catalog BCE (bert4rec/lightning.py:273-305)
+            self._model.core.set_loss("bce")
         self._optimizer_factory, self._lr_scheduler_factory = optimizer_factory, lr_scheduler_factory
         self._candidates_to_score = None
         self.fused_optimizer = fused_optimizer

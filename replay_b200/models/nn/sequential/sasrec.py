@@ -103,7 +103,8 @@ class SasRec(LightningModuleBase):
         super().__init__()
         self.save_hyperparameters()
         if loss_type not in ("CE", "BCE") or (loss_type == "BCE" and loss_sample_count is None):
-            raise NotImplementedError("Not supported loss_type")  # lightning.py:485 ; full-catalog BCE / SCE: no fused head
+            # lightning.py:485 ; SCE has no fused head; full-catalog BCE is selected on the core: _model.core.set_loss("bce")
+            raise NotImplementedError("Not supported loss_type")
         if negative_sampling_strategy not in {"global_uniform", "inbatch"}:
             raise AssertionError("negative_sampling_strategy must be 'global_uniform' or 'inbatch'")
         if loss_sample_count is not None and negative_sampling_strategy != "global_uniform":

@@ -1,6 +1,6 @@
 """Loss selectors with the reference's names and constructor arguments (replay/nn/loss/{ce,bce}.py).  They carry no
 computation: assigning one to ``SasRec.loss`` selects the fused CUDA head that implements it (full-catalog CE:
-rp_ce_head_*; sampled heads: rp_sampled_head_*).  Single positive label per position (multi-positive: NotImplementedError,
+rp_ce_head_*; full-catalog BCE: rp_bce_head_*; sampled heads: rp_sampled_head_*).  Single positive label per position (multi-positive: NotImplementedError,
 as in the reference's CE)."""
 from __future__ import annotations
 
@@ -31,6 +31,16 @@ class CE(_LossSpec):
         if kwargs:
             raise NotImplementedError(f"CrossEntropyLoss options {sorted(kwargs)} are not supported by the fused head")
         self.ignore_index = ignore_index
+
+
+class BCE(_LossSpec):
+    """replay/nn/loss/bce.py:10-95: ``BCEWithLogitsLoss(reduction="sum")`` over the whole catalog against the one-hot row of
+    each valid target, divided by the number of valid targets -> the fused full-catalog BCE head (rp_bce_head_*)."""
+    kind = "bce"
+
+    def __init__(self, **kwargs):
+        if kwargs:
+            raise NotImplementedError(f"BCEWithLogitsLoss options {sorted(kwargs)} are not supported by the fused head")
 
 
 class CESampled(_LossSpec):

@@ -38,7 +38,7 @@ class SasRec(torch.nn.Module):
 
     @property
     def loss(self):
-        """The reference's ``SasRec.loss`` attribute (model.py:181-197): assign ``CE`` / ``CESampled`` / ``BCESampled`` from
+        """The reference's ``SasRec.loss`` attribute (model.py:181-197): assign ``CE`` / ``BCE`` / ``CESampled`` / ``BCESampled`` from
         ``replay_b200.nn.loss`` to select the fused head."""
         return self._loss
 
@@ -46,7 +46,7 @@ class SasRec(torch.nn.Module):
     def loss(self, spec):
         if not hasattr(spec, "kind"):
             raise NotImplementedError(f"loss {type(spec).__name__} has no fused CUDA head (supported: CE, CEWeighted, LogOutCE, "
-                                      "LogOutCEWeighted, LogInCE, CESampled, BCESampled)")
+                                      "LogOutCEWeighted, LogInCE, BCE, CESampled, BCESampled)")
         self._loss = spec
         self.core.set_loss(spec.kind, **spec.engine_kwargs())
 

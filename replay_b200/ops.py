@@ -119,6 +119,42 @@ def ce_head_bwd(st: CEHeadState, hc, table, labels, n_valid, d_hc, d_table, bias
                                int(n_valid_hint), _ptr(st.ws), st.ws_bytes, _stream()), "rp_ce_head_bwd")
 
 
+class BCEHeadState:
+    """Buffers shared by rp_bce_head_fwd / rp_bce_head_bwd for one (capacity, n_items, d), d in {64, 128, 256}."""
+
+    def __init__(self, capacity: int, n_items: int, d: int, device, loss=None):
+        """``loss``: an fp32 [2] device buffer to write the loss into (the engines share the CE head's), else a new one."""
+        if d not in (64, 128, 256):
+            raise NotImplementedError(f"the full-catalog BCE head supports hidden sizes 64, 128 and 256 (got {d})")
+        self.capacity, self.n_items, self.d = capacity, n_items, d
+        self.ws_bytes = lib().rp_bce_head_workspace(capacity, n_items, d)
+        self.ws = torch.zeros(self.ws_bytes, device=device, dtype=torch.uint8)
+        self.loss = loss if loss is not None else torch.zeros(2, device=device, dtype=torch.float32)
+
+
+def bce_head_fwd(st: BCEHeadState, hc, table, labels, n_valid, d_hc, bias=None, n_valid_hint: int = 0):
+    """Full-catalog BCE: hc bf16 [capacity,d], table bf16 [I,d], labels int32 [capacity], n_valid int32 [1], bias fp32
+    [round_up(I,128)] or None.  d_hc (bf16 [capacity,d]) is final after this call.  Returns st.loss (fp32 [2]: mean loss,
+    1/n_valid) - a view that the next call overwrites."""
+    _need(hc, torch.bfloat16, "hc")
+    _need(table, torch.bfloat16, "table")
+    _need(labels, torch.int32, "labels")
+    _need(n_valid, torch.int32, "n_valid")
+    _need(d_hc, torch.bfloat16, "d_hc")
+    check(lib().rp_bce_head_fwd(_ptr(hc), _ptr(table), _ptr(bias), _ptr(labels), _ptr(n_valid), st.capacity, st.n_items, st.d,
+                                _ptr(st.loss), _ptr(d_hc), int(n_valid_hint), _ptr(st.ws), st.ws_bytes, _stream()),
+          "rp_bce_head_fwd")
+    return st.loss
+
+
+def bce_head_bwd(st: BCEHeadState, hc, table, labels, n_valid, d_table, bias=None, d_bias=None):
+    """d_table fp32 [>=I, d] (rows < I overwritten), d_bias fp32 [>=I] (iff bias; overwritten) of the last bce_head_fwd."""
+    _need(d_table, torch.float32, "d_table")
+    check(lib().rp_bce_head_bwd(_ptr(hc), _ptr(table), _ptr(bias), _ptr(labels), _ptr(n_valid), st.capacity, st.n_items, st.d,
+                                _ptr(st.loss), _ptr(d_table), _ptr(d_bias), _ptr(st.ws), st.ws_bytes, _stream()),
+          "rp_bce_head_bwd")
+
+
 def gemm(A, B, C, M, N, K, *, a_mn=False, b_mn=False, bias=None, act=0, residual=None, rowmask=None, drop_p=0.0,
          drop_offset=0, seed=0, seed_ptr=None, out_mode=0, split_k=1, gate=None, gate_scale=1.0, gate_mode=0, alpha=1.0,
          batch=1, inner=1, a_off=(0, 0, 0, 0, 0, 0), b_off=(0, 0, 0, 0, 0, 0), c_geom=None, rowmask_oo=0, C2=None,
